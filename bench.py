@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W    # the reference algorithm on host cores
     torchrun --nproc-per-node N ... bench.py --gpus N ...    # one rank per GPU (weak scaling)
+    python bench.py ... --dump-outputs DIR                   # also write what the last timed step computed
 
 A "step" is one Hebbian pretraining step of the reference loop (pretrain_hebbian_unsup_2d.py:181-196):
 zero_grad -> forward through the makehebbian()-converted UNet (22 Hebbian layers: conv forward +
@@ -57,7 +58,15 @@ def parse_args():
     ap.add_argument('--no-graph', action='store_true', help='launch every step eagerly')
     ap.add_argument('--fused-adam', action='store_true', help='(default) torch.optim.Adam(fused=True): one multi-tensor kernel for the optimiser step')
     ap.add_argument('--no-fused-adam', action='store_true', help='torch.optim.Adam with its default (for-each) implementation')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', default='', metavar='DIR',
+                    help='after the timed steps, write what the last one computed (network output, loss, parameters after the '
+                         'update) as DIR/<name>.npy in float32, for comparing two builds output for output')
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and a.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of --impl ours')
+    return a
 
 
 WORKLOADS = {
@@ -80,6 +89,22 @@ def peaks():
         return dict(hbm=float(d['hbm_gbs']), tf=float(d['bf16_tflops']), tf_sustained=float(d.get('bf16_tflops_sustained', d['bf16_tflops'])),
                     source='measured')
     return dict(hbm=6650.0, tf=1590.0, tf_sustained=1400.0, source='fallback')
+
+
+DUMP_MAX_ELEMS = 1 << 22        # per array (16 MB in float32); the three arrays of a dump stay under 64 MB
+
+
+def dump_outputs(path, arrays):
+    """Write each tensor as <path>/<name>.npy in float32.  A tensor of more than DUMP_MAX_ELEMS elements is written as
+    a fixed sample of them, flattened: the same seeded indices for every run, so two runs compare element for element."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randint(t.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(path, name + '.npy'), t.cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------
@@ -328,9 +353,10 @@ def roofline_from_rows(rows, prec, pk):
 
 
 def measure(args, workload, prec, B, steps, warmup, dev, world, rank, fuse=True, head_nchw=False, e2e=True, profile=True,
-            capture=False, layers_out='', fused_adam=None):
+            capture=False, layers_out='', fused_adam=None, dump_dir=''):
     """Build the workload on `dev`, time `steps` steps (HBM-resident inputs, CUDA events per step, L2 flushed between
-    steps, max over ranks) and, optionally, the end-to-end loop (pinned host batch in, loss out) and the per-layer profile."""
+    steps, max over ranks) and, optionally, the end-to-end loop (pinned host batch in, loss out) and the per-layer profile.
+    dump_dir: write the outputs of the last timed step there (dump_outputs)."""
     import torch.distributed as dist
     from hebb import _native
     from hebb.step import HebbianStepper
@@ -374,13 +400,26 @@ def measure(args, workload, prec, B, steps, warmup, dev, world, rank, fuse=True,
     with ClockSampler(dev.index or 0) as clk:
         sync_all()
         t_wall0 = time.perf_counter()
+        last = None
         for e0, e1 in evs:
             flush()
-            e0.record()
-            stepper.step(x, m)
+            if dump_dir:
+                last = None               # the previous step's outputs do not stay allocated through this step
+                e0.record()
+                last = stepper.step(x, m)
+            else:
+                e0.record()
+                stepper.step(x, m)
             e1.record()
         sync_all()
         t_wall = time.perf_counter() - t_wall0
+    if dump_dir and rank == 0:
+        out, loss = last
+        arrays = {'out': out} if loss is None else {'out': out, 'loss': loss}
+        arrays['params'] = torch.cat([p.detach().reshape(-1) for p in model.parameters()])
+        dump_outputs(dump_dir, arrays)
+        del out, loss, arrays
+    del last
     launches = _native.launch_count() - n0 + (stepper.graph_launches - g0)
     dev_ms = sum(e0.elapsed_time(e1) for e0, e1 in evs)
     t = torch.tensor([dev_ms], dtype=torch.float64, device=dev)
@@ -562,7 +601,7 @@ def run_ours(args):
     try:
         main = measure(args, args.workload, args.prec, B, args.steps, args.warmup, dev, world, rank, fuse=not args.no_fuse,
                        head_nchw=args.head_nchw, e2e=True, profile=not args.no_layer_profile, capture=want_graph(args.workload),
-                       layers_out=args.layers_out)
+                       layers_out=args.layers_out, dump_dir=args.dump_outputs)
     except Exception as e:
         if not want_graph(args.workload):
             raise
@@ -571,7 +610,8 @@ def run_ours(args):
         print(f'[bench] CUDA-graph capture failed ({graph_error}); falling back to eager launches', file=sys.stderr, flush=True)
         torch.cuda.synchronize()
         main = measure(args, args.workload, args.prec, B, args.steps, args.warmup, dev, world, rank, fuse=not args.no_fuse,
-                       head_nchw=args.head_nchw, e2e=True, profile=not args.no_layer_profile, capture=False, layers_out=args.layers_out)
+                       head_nchw=args.head_nchw, e2e=True, profile=not args.no_layer_profile, capture=False, layers_out=args.layers_out,
+                       dump_dir=args.dump_outputs)
 
     # ---- companions of the headline (single GPU, default workload only): the 3-D half of BASELINE's metric, the plain
     # drop-in number, the reference formulation on this GPU, the element-wise kernels ----

@@ -5,7 +5,6 @@ import json
 import os
 import sys
 
-import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -35,7 +34,8 @@ def pytest_collection_modifyitems(config, items):
 
 @pytest.fixture(scope='session')
 def golden():
-    return np.load(os.path.join(ROOT, 'tests', 'golden', 'hebb_golden.npz'))
+    import helpers
+    return helpers.load_golden('hebb_golden.npz')
 
 
 @pytest.fixture(scope='session')

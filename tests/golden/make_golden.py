@@ -3,10 +3,11 @@
 Run ONLY in the build container (needs /root/reference, which is not on the GPU
 box):  python tests/golden/make_golden.py
 The reference modules are imported unchanged under an alias; nothing is copied.
-Each case stores the inputs (x, W, bias, hyper-parameters) and what the
-reference produced (y, argmax winners, delta_w, grad after local_update, W
+Each case stores what the reference produced (y, argmax winners, delta_w, W
 after N optimiser steps), so both the oracle and the CUDA path can be checked
-on a box without the reference.
+without the reference.  The inputs (x, W, bias) come from one seeded generator
+per file and are not stored: tests/helpers.py::load_golden draws them again,
+and derives grad after local_update (= -delta_w).
 """
 import importlib.util
 import io
@@ -22,6 +23,8 @@ import torch.nn as nn
 REF = os.environ.get('HEBB_REFERENCE', '/root/reference')
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.dont_write_bytecode = True
+sys.path.insert(0, os.path.dirname(HERE))
+import helpers  # noqa: E402  (tests/helpers.py: load_golden re-creates the inputs this script does not store)
 
 
 def load_reference():
@@ -58,6 +61,17 @@ CONVT_CASES = [
     ('t3d_2x2x2_s2', 3, 2, 8, 4, 2, 2, (3, 4, 5), 50.0),
     ('t3d_40co',    3, 1, 6, 40, 2, 2, (2, 3, 3), 5.0),    # > PARALLEL_CHANNELS out channels
 ]
+
+
+def stored(out, redrawn, drawn_again):
+    """The arrays of `out` that tests/helpers.py::load_golden does not re-create.  drawn_again: the inputs as
+    load_golden draws them (helpers._draw_r1 / _draw_r2), which must equal the ones the reference ran on."""
+    mine = {k: v for k, v in out.items() if k.rsplit('/', 1)[1] in ('x', 'w', 'b', 'xs', 'w0')}
+    bad = sorted(set(mine) ^ set(drawn_again)) + [k for k in mine if k in drawn_again and
+                                                  not np.array_equal(mine[k], drawn_again[k].numpy())]
+    if bad:
+        raise RuntimeError(f'tests/helpers.py draws other inputs than this script for {bad[:5]}: update its case order')
+    return {k: v for k, v in out.items() if k.rsplit('/', 1)[1] not in redrawn}
 
 
 def main():
@@ -215,7 +229,7 @@ def main():
         meta[name] = dict(kind='contrastive', nd=nd, B=B, Cin=Cin, Cout=Cout, kernel=3, stride=1, padding=1,
                           spatial=list(spatial), bias=bias, uniformity=uniformity, contrast=contrast)
 
-    np.savez_compressed(os.path.join(HERE, 'hebb_golden.npz'), **out)
+    np.savez_compressed(os.path.join(HERE, 'hebb_golden.npz'), **stored(out, ('x', 'w', 'b', 'xs', 'w0', 'grad'), helpers._draw_r1(meta)))
 
     # ---- makehebbian structure on the reference test's toy net (tests/test_makehebbian.py:5-39)
     class Net(nn.Module):
@@ -402,7 +416,7 @@ def round2_goldens():
         out[name + '/x'], out[name + '/w'] = x.numpy(), layer.weight.detach().contiguous().numpy()
         out[name + '/y'], out[name + '/dw1'] = y.detach().numpy(), layer.delta_w.clone().contiguous().numpy()
         meta[name] = dict(kind='hpca_t', nd=nd, B=B, Cin=Cin, Cout=Cout, spatial=list(sp))
-    np.savez_compressed(os.path.join(HERE, 'hebb_golden_r2.npz'), **out)
+    np.savez_compressed(os.path.join(HERE, 'hebb_golden_r2.npz'), **stored(out, ('x', 'w', 'b', 'xs', 'w0'), helpers._draw_r2(meta)))
 
     with contextlib.redirect_stdout(io.StringIO()):
         r2 = _load_file(os.path.join(REF, 'models/networks_2d/unet.py'), 'ref_unet2d')

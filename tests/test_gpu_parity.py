@@ -17,7 +17,7 @@ from hebb.makehebbian import makehebbian
 from hebb.step import HebbianStepper, hebbian_layers
 import workloads
 from oracle import hebb_oracle as O
-from helpers import record
+from helpers import load_golden, record
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -792,7 +792,7 @@ def test_hpca_transposed_vs_reference_golden(golden, name):
 
 
 # ---- round 2: tensor-core-shaped 100-step drift, non-Identity act, network training loop, NCCL exchange ----
-G2 = np.load(os.path.join(ROOT, 'tests', 'golden', 'hebb_golden_r2.npz'))
+G2 = load_golden('hebb_golden_r2.npz')
 STEPS = json.load(open(os.path.join(ROOT, 'tests', 'golden', 'network_steps_golden.json')))
 
 

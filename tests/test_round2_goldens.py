@@ -15,10 +15,10 @@ import torch.multiprocessing as mp
 
 import workloads
 from oracle import hebb_oracle as O
-from helpers import digest_err
+from helpers import digest_err, load_golden
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-G2 = np.load(os.path.join(ROOT, 'tests', 'golden', 'hebb_golden_r2.npz'))
+G2 = load_golden('hebb_golden_r2.npz')
 STEPS = json.load(open(os.path.join(ROOT, 'tests', 'golden', 'network_steps_golden.json')))
 G2B = np.load(os.path.join(ROOT, 'tests', 'golden', 'hebb_golden_r2b.npz'))
 META2B = json.load(open(os.path.join(ROOT, 'tests', 'golden', 'hebb_golden_r2b_meta.json')))
